@@ -4,12 +4,14 @@ ray-samples/sec).  One "step" = one Trainer.step(): K1 sampling -> K4 fused PE+M
 input-gradient / losses / double back-prop -> K5 -> [C1 all-reduce] -> K6 AdamW+re-pack.
 
   python bench.py --gpus N --steps K --warmup W [--impl reference] [--precision bf16x3|bf16|fp32]
-                  [--workload default|scannet|c4|c5]
+                  [--workload default|scannet|c4|c5] [--dump-outputs DIR]
 
 Prints ONE JSON line (contract in the task statement): metric/value/unit (device-resident inputs),
 e2e (public API with host frames, H2D + D2H inside the timed region), roofline (dominant kernel,
 CUDA-event timed inside the library), cpu_baseline (oracle port on the host cores), clocks.
-`--impl reference` times the CPU port of the reference's own step instead (rank 0 only)."""
+`--impl reference` times the CPU port of the reference's own step instead (rank 0 only).
+`--dump-outputs DIR` writes what the timed step path computes as DIR/<name>.npy (float32, at most 64 MB); the inputs are
+seeded, so two builds run with the same arguments can be compared output for output."""
 import argparse
 import json
 import os
@@ -44,6 +46,58 @@ WORKLOADS = {
                  name="get_sdf_grid 200^3 lattice (8.0 M points, forward-only K2, lattice generated in-kernel), 256x(2+2) MLP"),
 }
 PEAKS_FALLBACK = dict(hbm_gbs=6650.0, bf16_tflops=1590.0, bf16_tflops_sustained=1400.0)
+DUMP_MAX_ELEMENTS = 1 << 22          # per array (16 MB of float32); a dump holds at most three arrays this large
+
+
+def host_copy(t):
+    """float32 numpy copy of a device or host tensor; an array above DUMP_MAX_ELEMENTS is cut to a fixed seeded sample
+    of its flattened elements (the same positions in every run of the same workload)."""
+    import numpy as np
+    a = t.detach().float().cpu().numpy().copy()
+    if a.size > DUMP_MAX_ELEMENTS:
+        idx = np.sort(np.random.default_rng(0).choice(a.size, DUMP_MAX_ELEMENTS, replace=False))
+        a = a.reshape(-1)[idx]
+    return a
+
+
+def make_trainer(dev, wl, precision, rank=0, world=1, dist=None):
+    """The seeded Trainer of the timed path with this rank's keyframe shard (frames rank, rank + world, ...) resident."""
+    import numpy as np
+    from isdf.modules import trainer as trainer_mod
+    np.random.seed(1 + rank)
+    torch.manual_seed(1 + rank)
+    tr = trainer_mod.Trainer(dev, make_config(wl, precision, "fast"), incremental=True)
+    if dist is not None:                            # identical replicas: broadcast rank 0's parameters
+        dist.broadcast(tr.sdf_map.flat_parameters(), 0)
+    for i in range(wl["keyframes"]):
+        tr.last_is_keyframe = True
+        tr.add_data(tr.get_data([rank + i * world]))
+    return tr
+
+
+def reproducible_step(dev, wl, precision, n_steps=3):
+    """What the timed step path returns and leaves in the model, from a state every run reproduces: a Trainer seeded and
+    loaded like the timed one takes n_steps steps (a new layout's first step runs eagerly, the second captures the CUDA
+    graph, the third replays it as every timed step does) and its last step is recorded.  The timed trainer's own last
+    step is not reproducible: the library sums gradients and losses with float atomics, so two runs of one build differ in
+    the last bits every step, and over hundreds of steps AdamW and the loss-weighted keyframe window grow that into
+    visibly different trajectories."""
+    tr = make_trainer(dev, wl, precision)
+    for _ in range(n_steps):
+        losses, _ = tr.step(sync=False)
+    torch.cuda.synchronize(dev)
+    out = {k: host_copy(v) for k, v in losses.items()}
+    out.update(sdf=host_copy(tr.last_sdf), loss_mat=host_copy(tr.last_loss_mat),
+               params=host_copy(tr.sdf_map.flat_parameters()), frame_avg_losses=host_copy(tr.frames.frame_avg_losses))
+    return out
+
+
+def write_dump(out_dir, arrays):
+    import numpy as np
+    assert sum(a.nbytes for a in arrays.values()) <= 64 << 20
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 def load_peaks():
@@ -253,10 +307,11 @@ def run_grid_bench(args, wl, dev, rank, world, dist):
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     e0.record()
     for _ in range(args.steps):
-        tr.get_sdf_grid()
+        grid = tr.get_sdf_grid()
     e1.record()
     torch.cuda.synchronize(dev)
     ms = e0.elapsed_time(e1)
+    dump = {"sdf_grid": host_copy(grid)} if args.dump_outputs else None
     clocks = sampler.stop() if rank == 0 else None
     t = torch.tensor([ms], device=dev, dtype=torch.float64)
     if dist is not None:
@@ -308,6 +363,8 @@ def run_grid_bench(args, wl, dev, rank, world, dist):
                        "api": "Trainer.get_sdf_grid() + D2H of the [200,200,200] grid into pinned memory"},
                "gpu_launches": launches_per_step * args.steps, "roofline": roof, "cpu_baseline": None}
         print(json.dumps(out))
+    if dump is not None:
+        write_dump(args.dump_outputs, dump)
 
 
 def main():
@@ -320,7 +377,13 @@ def main():
                     choices=["bf16x3g", "bf16x3", "bf16", "fp32"])
     ap.add_argument("--workload", default="default", choices=sorted(WORKLOADS))
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the step's outputs (losses, sdf, loss matrix, parameters and "
+                         "per-keyframe losses after the step; see reproducible_step) or, for the grid workload, the last "
+                         "timed sdf grid as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.dump_outputs and (args.impl == "reference" or int(os.environ.get("WORLD_SIZE", 1)) > 1):
+        ap.error("--dump-outputs records the B200 path of a single process")
     wl = WORKLOADS[args.workload]
     rank = int(os.environ.get("RANK", 0))
     local_rank = int(os.environ.get("LOCAL_RANK", 0))
@@ -343,30 +406,16 @@ def main():
         import torch.distributed as dist
         dist.init_process_group("nccl", device_id=dev)
     say("process group ready")
-    import __graft_entry__ as ge
-    if rank == 0:
-        ge.build()
-    if dist is not None:
-        dist.barrier()
-    say("library built")
+    # the library __graft_entry__.build() compiled; the benchmark itself writes nothing into the tree
+    from isdf_b200 import _lib
+    _lib.load()
+    say("library loaded")
     if args.workload == "grid":
         run_grid_bench(args, wl, dev, rank, world, dist)
         if dist is not None:
             dist.destroy_process_group()
         return
-    from isdf.modules import trainer as trainer_mod
-    import numpy as np
-
-    np.random.seed(1 + rank)
-    torch.manual_seed(1 + rank)
-    cfg = make_config(wl, args.precision, "fast")
-    tr = trainer_mod.Trainer(dev, cfg, incremental=True)
-    if world > 1:                                   # identical replicas: broadcast rank 0's parameters
-        dist.broadcast(tr.sdf_map.flat_parameters(), 0)
-    # keyframe shard of this rank: frames k = rank, rank + world, ...
-    for i in range(wl["keyframes"]):
-        tr.last_is_keyframe = True
-        tr.add_data(tr.get_data([rank + i * world]))
+    tr = make_trainer(dev, wl, args.precision, rank, world, dist)
     say("keyframes resident")
     S = wl["n_strat"] + wl["n_surf"]
     rays_per_step = wl["n_rays"] * 5
@@ -571,6 +620,8 @@ def main():
                "sample": "5 steps of %d rays x %d samples after 1 warm-up; %s" % (n_r * 5, S, what),
                "iters_per_sec": 5 / dt, "ms_per_step_median": 1000.0 * statistics.median(per)}
 
+    if args.dump_outputs:           # before the result line, which stays the last line on stdout
+        write_dump(args.dump_outputs, reproducible_step(dev, wl, args.precision))
     if rank == 0:
         out = {"metric": "train ray-samples/sec", "value": value, "unit": "ray-samples/s",
                "iters_per_sec": world * args.steps / (ms_max / 1000.0) / world,
