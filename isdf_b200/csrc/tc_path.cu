@@ -313,6 +313,15 @@ int tc_forward_grid(isdfb_ctx* ctx, const float* lin, int dim, const float* scal
   return tc_forward_impl(ctx, nullptr, nullptr, 0.f, (int64_t)dim * dim * dim, sdf, nullptr, st, &g);
 }
 
+// Grid of the wave-1 weight-gradient launch of a two-wave chunk (tiles = num_sms + rest): the CTAs the partial wave 2
+// leaves idle, but never fewer than one CTA per job -- tc_dw_kernel maps CTA b to job b % n_jobs, so a smaller grid
+// would leave jobs n_jobs-grid.. without a CTA and their gradient over the first num_sms tiles would be lost.  The
+// launch and the exchange's expected-arrival counts both take the grid from here.
+static inline int dw_wave1_grid(const TcState* tc, int rest) {
+  const int idle = tc->num_sms - rest;
+  return idle > tc->dw.n_jobs ? idle : tc->dw.n_jobs;
+}
+
 int tc_train(isdfb_ctx* ctx, const float* pc, const float* z_vals, const float* depth_sample, const float* dirs_C,
              const float* T_WC_sample, const float* norm_sample, const float* noise, const uint8_t* ray_valid,
              int64_t n_rays, int32_t S, const isdfb_loss_cfg* loss, float* sdf, float* grad, float* loss_mat,
@@ -335,7 +344,7 @@ int tc_train(isdfb_ctx* ctx, const float* pc, const float* z_vals, const float* 
       const int tiles = (int)((nc + TC_TILE - 1) / TC_TILE);
       if (tiles > tc->num_sms && tiles < 2 * tc->num_sms && two_wave_ok) {
         const int rest = tiles - tc->num_sms;
-        plan(tc->num_sms - rest > 14 ? tc->num_sms - rest : 14, tc->num_sms);
+        plan(dw_wave1_grid(tc, rest), tc->num_sms);
         plan(tc->num_sms, rest);
       } else {
         plan(tc->num_sms, tiles);
@@ -379,7 +388,7 @@ int tc_train(isdfb_ctx* ctx, const float* pc, const float* z_vals, const float* 
       ISDFB_CUDA_OK(ctx, cudaStreamWaitEvent(tc->side, tc->ev_fork, 0));
       d.tile0 = 0; d.n_tiles = tc->num_sms;
       const int rest = total_tiles - tc->num_sms;
-      rc = tc_dw_launch(ctx, d, dw_passes_of(ctx), tc->num_sms - rest > 14 ? tc->num_sms - rest : 14, tc->side);
+      rc = tc_dw_launch(ctx, d, dw_passes_of(ctx), dw_wave1_grid(tc, rest), tc->side);
       if (rc) return rc;
       ISDFB_CUDA_OK(ctx, cudaEventRecord(tc->ev_join, tc->side));
       a.tile0 = tc->num_sms; a.n_tiles = rest;

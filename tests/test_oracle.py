@@ -193,6 +193,58 @@ def test_adamw_matches_torch():
         assert torch.allclose(p, gold[it], atol=1e-6, rtol=1e-6)
 
 
+LOSS_SETTINGS = [   # (id, n_freqs, block, cfg overrides, batch kind): the settings tests/test_gpu_zz_train_geometry.py uses
+    ("orien_loss", 6, 2, dict(orien_loss=True), "ray"),
+    ("grad_weight_0", 6, 2, dict(grad_weight=0.0), "ray"),
+    ("eik_weight_0", 6, 2, dict(eik_weight=0.0), "ray"),
+    ("grad_and_eik_0", 6, 2, dict(grad_weight=0.0, eik_weight=0.0), "ray"),
+    ("franka_E465_b3", 11, 3, dict(trunc_weight=30.0, trunc_distance=0.1, noise_std=0.025, dist_behind_surf=0.01), "franka"),
+    ("scale_input_0.4_E381", 9, 2, dict(scale_input=0.4), "ray"),
+    ("pc_bound_E381", 9, 2, dict(bounds_method="pc"), "pc"),
+]
+
+
+@pytest.mark.parametrize("tag,n_freqs,block,over,kind", LOSS_SETTINGS, ids=[s[0] for s in LOSS_SETTINGS])
+def test_oracle_formulations_agree_at_every_loss_setting(tag, n_freqs, block, over, kind):
+    """The closed-form adjoints of step_sweeps (orien_loss, switched-off terms, franka truncation, large PE arguments,
+    the 'pc' bound) equal autograd of the reference formulation in fp64.  grad_weight 0 runs without normals, as the
+    Trainer does."""
+    cfg = O.default_cfg(n_freqs=n_freqs, block=block, n_strat=8, n_surf=8, **dict(dict(noise_std=0.08), **over))
+    sd = C.golden_weights(7, E=3 + 42 * n_freqs, block=block, gain=1.2)
+    layers = [(w.double(), b.double()) for w, b in O.layers_from_state_dict(sd, block)]
+    if kind == "pc":
+        batch, noise = C.loss_batch_pc(19, 6, S=16)
+    else:
+        batch, noise = C.loss_batch(19, 6, S=16, dist_behind=cfg["dist_behind_surf"])
+    batch = {k: v.double() for k, v in batch.items()}
+    if cfg["grad_weight"] == 0:
+        batch["norm_sample"] = None
+    a = O.step_autograd(layers, batch, cfg, noise.double())
+    s = O.step_sweeps(layers, batch, cfg, noise.double())
+    assert (a["sdf"] - s["sdf"]).abs().max() < 1e-12 and (a["g"] - s["g"]).abs().max() < 1e-12
+    assert set(a["losses"]) == set(s["losses"])
+    assert ("grad_loss" in s["losses"]) == (cfg["grad_weight"] != 0)
+    assert ("eikonal_loss" in s["losses"]) == (cfg["eik_weight"] != 0)
+    for k in a["losses"]:
+        assert abs(float(a["losses"][k] - s["losses"][k])) <= 1e-12 * max(1.0, abs(float(a["losses"][k]))), k
+    for ga, gs in zip(a["grads"], s["grads"]):
+        assert float(ga.abs().max()) > 0
+        assert (ga - gs).abs().max() <= 1e-10 * max(1.0, float(ga.abs().max()))
+
+
+def test_step_sweeps_is_device_generic():
+    """step_sweeps builds every constant on the device of its inputs (the GPU tests run the fp64 oracle there): on a
+    'meta' batch it must get through without touching a CPU tensor."""
+    cfg = O.default_cfg(noise_std=0.08, n_strat=8, n_surf=8, transform=C.rigid_transform(9).double())
+    sd = C.golden_weights(7)
+    batch, noise = C.loss_batch(19, 4, S=16)
+    meta = torch.device("meta")
+    layers = [(w.double().to(meta), b.double().to(meta)) for w, b in O.layers_from_state_dict(sd, 2)]
+    b = {k: v.double().to(meta) for k, v in batch.items()}
+    out = O.step_sweeps(layers, b, dict(cfg, transform=cfg["transform"].to(meta)), noise.double().to(meta))
+    assert out["sdf"].device == meta and all(g.device == meta for g in out["grads"])
+
+
 @pytest.mark.parametrize("n_freqs,hidden,block", [(6, 512, 4), (9, 256, 2), (11, 256, 3)])
 def test_oracle_formulations_agree_at_other_model_shapes(n_freqs, hidden, block):
     """The shapes of BASELINE configs[4] and of the realsense / franka configs (SURVEY.md appendix A): the explicit
