@@ -245,6 +245,49 @@ def test_step_sweeps_is_device_generic():
     assert out["sdf"].device == meta and all(g.device == meta for g in out["grads"])
 
 
+@pytest.mark.parametrize("n_freqs,block,tr,scale_input", [(6, 2, None, 0.05937489), (6, 3, 9, 0.05937489),
+                                                          (9, 2, 9, 0.4), (11, 3, 5, 0.05937489)])
+def test_sdf_and_grad_equals_step_sweeps_fp64(n_freqs, block, tr, scale_input):
+    """sdf_and_grad (autograd over sdf_forward; the oracle of the forward-only and input-gradient programs) equals the
+    sdf and g of the explicit sweeps, with noise, a rigid PE transform and a large scale_input."""
+    cfg = O.default_cfg(n_freqs=n_freqs, block=block, noise_std=0.3, scale_input=scale_input,
+                        transform=C.rigid_transform(tr).double() if tr else None, n_strat=8, n_surf=8)
+    sd = C.golden_weights(13, E=O.embedding_size(n_freqs), block=block, gain=1.2)
+    layers = [(w.double(), b.double()) for w, b in O.layers_from_state_dict(sd, block)]
+    batch, noise = C.loss_batch(23, 5, S=16)
+    batch = {k: v.double() for k, v in batch.items()}
+    ref = O.step_sweeps(layers, batch, cfg, noise.double())
+    sdf, g = O.sdf_and_grad(layers, batch["pc"], cfg, noise.double())
+    assert sdf.shape == (5, 16) and g.shape == (5, 16, 3) and sdf.dtype == torch.float64
+    assert float((sdf - ref["sdf"]).abs().max()) < 1e-12 and float((g - ref["g"]).abs().max()) < 1e-12
+    sdf0, g0 = O.sdf_and_grad(layers, batch["pc"], cfg)               # noise shifts sdf only
+    assert torch.allclose(sdf - sdf0, noise.double() * 0.3 * cfg["scale_output"], rtol=0, atol=1e-12)
+    assert torch.equal(g, g0)
+
+
+@pytest.mark.parametrize("tag,seed,gain,tr", [("g1", 21, 1.0, None), ("g2_rigid", 22, 2.0, 6)])
+def test_sdf_and_grad_matches_reference(tag, seed, gain, tr):
+    gold = load("sdfmap.pt")[tag]
+    sd = C.golden_weights(seed, gain=gain)
+    for dt, tol_s, tol_g in ((torch.float32, 2e-6, 2e-5), (torch.float64, 5e-6, 1e-4)):
+        layers = [(w.to(dt), b.to(dt)) for w, b in O.layers_from_state_dict(sd, 2)]
+        cfg = O.default_cfg(transform=C.rigid_transform(tr).to(dt) if tr else None)
+        x = ((torch.rand(96, 3, generator=C.gen(12)) - 0.5) * torch.tensor([12.0, 4.0, 12.0])).to(dt)
+        sdf, g = O.sdf_and_grad(layers, x, cfg)
+        assert float((sdf - gold["sdf"]).abs().max() / gold["sdf"].abs().max()) < tol_s
+        assert float((g - gold["grad"]).abs().max() / gold["grad"].abs().max()) < tol_g
+
+
+def test_sdf_and_grad_is_device_generic():
+    meta = torch.device("meta")
+    cfg = O.default_cfg(n_freqs=9, transform=C.rigid_transform(9).double().to(meta))
+    sd = C.golden_weights(7, E=O.embedding_size(9))
+    layers = [(w.double().to(meta), b.double().to(meta)) for w, b in O.layers_from_state_dict(sd, 2)]
+    x = torch.empty(4, 7, 3, dtype=torch.float64, device=meta)
+    sdf, g = O.sdf_and_grad(layers, x, cfg, torch.empty(4, 7, dtype=torch.float64, device=meta))
+    assert sdf.device == meta and g.device == meta and sdf.shape == (4, 7) and g.shape == (4, 7, 3)
+
+
 @pytest.mark.parametrize("n_freqs,hidden,block", [(6, 512, 4), (9, 256, 2), (11, 256, 3)])
 def test_oracle_formulations_agree_at_other_model_shapes(n_freqs, hidden, block):
     """The shapes of BASELINE configs[4] and of the realsense / franka configs (SURVEY.md appendix A): the explicit
