@@ -26,14 +26,6 @@
 #include "tc_chain.cuh"
 #include "pe_loss.cuh"
 
-// Timing ablations (ISDFB_ABLATE, tools/ablate*.sh) are a DEV build option: compiled in only with -DISDFB_DEV_ABLATE.
-// In the product build every test below is a compile-time false -- they were 5 predicate tests (LOP3 + ISETP + BRA)
-// per 8-element sub-piece of every epilogue, ~10 % of the issued instructions.
-#ifdef ISDFB_DEV_ABLATE
-#define ABL(flags, bit) ((flags) & (bit))
-#else
-#define ABL(flags, bit) 0
-#endif
 #define EPI_WARPS 16
 #define EPI_THREADS (EPI_WARPS * 32)
 #define NUM_THREADS (EPI_THREADS + 128)   // + one helper warpgroup: MMA issuer, weight producer, two idle warps
@@ -84,7 +76,6 @@ struct EpiT {                       // per-thread / per-tile constants (thread o
   size_t dwl_stride, aux_stride, sig_stride;
   int p, kcol;                      // kcol = 16 jg
   int c0;                           // first K chunk of this CTA's rotated order (rot_kstep)
-  int ablate;
 };
 struct EpiOps { uint4 s, b0, b1, e0, e1; };   // side-array operands of one sub-piece (e0/e1: own embedding values, S2_END)
 struct EpiStepPtrs {                  // per-step pointers (thread offsets included)
@@ -97,7 +88,6 @@ struct EpiStepPtrs {                  // per-step pointers (thread offsets inclu
   const float *bias, *wout;
   float* hlast;
   const float* e32;                   // this thread's slice of the fp32 embedding side array (same offsets as aux)
-  int ablate;
   int flags;                          // TcStep::flags (STF_*)
   int ecol0;                          // EPI_S2_END: first internal embedding column of this step's outputs (256 * eh)
 };
@@ -111,11 +101,11 @@ template <int kPasses, bool kLean>
 __device__ __forceinline__ void put8(const EpiT& T, const float* x, int c, int h, bool to_a, int dwl_arr) {
   uint4 hi, lo;
   if (kPasses == 3 && (to_a || !kLean)) split8(x, hi, lo); else hi = pack8_hi(x);
-  if (to_a && !ABL(T.ablate, 32)) {
+  if (to_a) {
     *reinterpret_cast<uint4*>(T.a_hi + sub_a(c, h)) = hi;
     if (kPasses == 3) *reinterpret_cast<uint4*>(T.a_lo + sub_a(c, h)) = lo;
   }
-  if (dwl_arr >= 0 && !ABL(T.ablate, 1)) {
+  if (dwl_arr >= 0) {
     const size_t off = (size_t)dwl_arr * T.dwl_stride + sub_d(c, h);
     *reinterpret_cast<uint4*>(T.dwl_hi + off) = hi;
     if (kPasses == 3 && !kLean) *reinterpret_cast<uint4*>(T.dwl_lo + off) = lo;
@@ -124,7 +114,6 @@ __device__ __forceinline__ void put8(const EpiT& T, const float* x, int c, int h
 
 template <int EPI, int kPasses, bool kLean>
 __device__ __forceinline__ void epi_load(const EpiStepPtrs& P, bool l_is_cat, int c, int h, EpiOps& o) {
-  if (ABL(P.ablate, 8)) return;
   auto ld = [&](const void* q) -> uint4 { return ld_stream(q); };   // read-once side state: never allocates in L1
   if (EPI == EPI_S2 || EPI == EPI_S3 || EPI == EPI_S3_LAST || EPI == EPI_S4)
     o.s = ld(P.sigp + sub_a(c, h));
@@ -150,7 +139,7 @@ __device__ __forceinline__ void epi_load(const EpiStepPtrs& P, bool l_is_cat, in
 
 struct EpiAcc { float raw_acc, gx, gy, gz; };
 
-// Per-CTA rotation of the K order of every product (args.stagger): CTA b walks the four 64-column K chunks
+// Per-CTA rotation of the K order of every product: CTA b walks the four 64-column K chunks
 // starting at chunk (b/4)%4 and the four K steps inside a chunk starting at b%4.  All CTAs stream the SAME
 // weight images from L2 at the same pace; without the rotation the 148 SMs ask the same L2 lines for the same
 // 8 KB block at the same moment and queue behind each other (measured: 12 k cycles per step for the weight
@@ -170,10 +159,8 @@ __device__ __forceinline__ void epi_sub(const TcChainArgs& args, const EpiT& T, 
       const float4 pa = ld4(P.part_out + sub_x(c, h)), pb = ld4(P.part_out + sub_x(c, h) + 512);
       v[0] += pa.x; v[1] += pa.y; v[2] += pa.z; v[3] += pa.w; v[4] += pb.x; v[5] += pb.y; v[6] += pb.z; v[7] += pb.w;
     }
-    if (!ABL(T.ablate, 2)) {
-      st4(P.part_out + sub_x(c, h), v[0], v[1], v[2], v[3]);
-      st4(P.part_out + sub_x(c, h) + 512, v[4], v[5], v[6], v[7]);
-    }
+    st4(P.part_out + sub_x(c, h), v[0], v[1], v[2], v[3]);
+    st4(P.part_out + sub_x(c, h) + 512, v[4], v[5], v[6], v[7]);
   } else if (EPI == EPI_S1 || EPI == EPI_S1_LAST) {
     const float4 ba = ld4(P.bias + k0), bb = ld4(P.bias + k0 + 4);
     float z[8] = {v[0] + ba.x, v[1] + ba.y, v[2] + ba.z, v[3] + ba.w, v[4] + bb.x, v[5] + bb.y, v[6] + bb.z, v[7] + bb.w};
@@ -182,20 +169,15 @@ __device__ __forceinline__ void epi_sub(const TcChainArgs& args, const EpiT& T, 
       z[4] += __uint_as_float(o.b1.x); z[5] += __uint_as_float(o.b1.y); z[6] += __uint_as_float(o.b1.z); z[7] += __uint_as_float(o.b1.w);
     }
     float hh[8], sg[8];
-    if (ABL(T.ablate, 16)) {
 #pragma unroll
-      for (int t = 0; t < 8; ++t) { hh[t] = fmaxf(z[t], 0.f); sg[t] = z[t] > 0.f ? 1.f : 0.f; }
-    } else {
-#pragma unroll
-      for (int t = 0; t < 8; ++t) softplus100_fast(z[t], hh[t], sg[t]);
-    }
-    if (store_state && !ABL(T.ablate, 4)) *reinterpret_cast<uint4*>(P.sigw + sub_a(c, h)) = pack_unorm16x8(sg);
+    for (int t = 0; t < 8; ++t) softplus100_fast(z[t], hh[t], sg[t]);
+    if (store_state) *reinterpret_cast<uint4*>(P.sigw + sub_a(c, h)) = pack_unorm16x8(sg);
     if (EPI == EPI_S1) {
       put8<kPasses, kLean>(T, hh, c, h, true, (train && l + 1 < args.L) ? args.arr_yh + l + 1 : -1);
     } else {
       const float4 wa = ld4(P.wout + k0), wb = ld4(P.wout + k0 + 4);
       const float ww[8] = {wa.x, wa.y, wa.z, wa.w, wb.x, wb.y, wb.z, wb.w};
-      if (train && !ABL(T.ablate, 2)) {
+      if (train) {
         st4(P.hlast + sub_x(c, h), hh[0], hh[1], hh[2], hh[3]);
         st4(P.hlast + sub_x(c, h) + 512, hh[4], hh[5], hh[6], hh[7]);
       }
@@ -213,7 +195,6 @@ __device__ __forceinline__ void epi_sub(const TcChainArgs& args, const EpiT& T, 
     for (int t = 0; t < 8; ++t) v[t] *= sg[t];
     put8<kPasses, kLean>(T, v, c, h, true, train ? args.arr_xd + l : -1);
   } else if (EPI == EPI_S2_END) {
-    if (ABL(T.ablate, 64)) { acc.gx += v[0]; return; }
     // PE Jacobian in the internal column order (tc_common.cuh): columns (2i, 2i+1) = (sin, cos) of pair i, so
     // d e / d xb = (cos, -sin) is thread-local:  g_xs += D_d 2^f (cos a_sin - sin a_cos);  x y z follow the pairs
     const int two_half = 2 * ISDFB_NDIRS * args.pe.n_freqs;
@@ -257,13 +238,11 @@ __device__ __forceinline__ void epi_sub(const TcChainArgs& args, const EpiT& T, 
       v[t] = v[t] * sg[t];                 // abar = dbar * sigma
     }
     if (EPI == EPI_S3) {
-      if (!ABL(T.ablate, 2)) {
-        if (kLean) {
-          *reinterpret_cast<uint4*>(P.zb2h + sub_a(c, h)) = pack8_hi(zb);
-        } else {
-          st4(P.zb2 + sub_x(c, h), zb[0], zb[1], zb[2], zb[3]);
-          st4(P.zb2 + sub_x(c, h) + 512, zb[4], zb[5], zb[6], zb[7]);
-        }
+      if (kLean) {
+        *reinterpret_cast<uint4*>(P.zb2h + sub_a(c, h)) = pack8_hi(zb);
+      } else {
+        st4(P.zb2 + sub_x(c, h), zb[0], zb[1], zb[2], zb[3]);
+        st4(P.zb2 + sub_x(c, h) + 512, zb[4], zb[5], zb[6], zb[7]);
       }
       put8<kPasses, kLean>(T, v, c, h, true, (l + 1 < args.L) ? args.arr_ya + l + 1 : -1);
     } else {
@@ -297,8 +276,8 @@ __device__ __forceinline__ void epi_sub(const TcChainArgs& args, const EpiT& T, 
   }
 }
 
-// one whole step of the epilogue for this thread (8 sub-pieces), operands fetched one sub-piece ahead
-template <int EPI, int kPasses, int kWide, bool kLean, int kNE>
+// one whole step of the epilogue for this thread (8 sub-pieces), operands fetched two sub-pieces ahead
+template <int EPI, int kPasses, bool kLean, int kNE>
 __device__ __forceinline__ void epi_step(const TcChainArgs& args, const EpiT& T, const EpiStepPtrs& P, ChainSmemTail* tail,
                                          uint32_t d_tmem, uint32_t n, int l, bool train, bool store_state, bool last_step,
                                          float sbar, EpiAcc& acc, int lane) {
@@ -322,54 +301,28 @@ __device__ __forceinline__ void epi_step(const TcChainArgs& args, const EpiT& T,
       for (int c = 0; c < 4; ++c) mbar_arrive(smem_u32(&tail->a_ready[c]));
     }
   }
-  if (kWide) {
-    // operands of BOTH sub-pieces of the next chunk are requested before this chunk is processed: two sub-pieces
-    // of lead on the side-state loads (L2 latency under load exceeds one) at the price of two more operand sets
-    epi_load<EPI, kPasses, kLean>(P, l_is_cat, T.c0, 1, ob);
+  // operands of BOTH sub-pieces of the next chunk are requested before this chunk is processed: two sub-pieces
+  // of lead on the side-state loads (L2 latency under load exceeds one) at the price of two more operand sets
+  epi_load<EPI, kPasses, kLean>(P, l_is_cat, T.c0, 1, ob);
 #pragma unroll 1
-    for (int ci = 0; ci < 4; ++ci) {
-      const int c = (ci + T.c0) & 3;
-      EpiOps na = oa, nb = ob;
-      if (ci < 3) {
-        epi_load<EPI, kPasses, kLean>(P, l_is_cat, (c + 1) & 3, 0, na);
-        epi_load<EPI, kPasses, kLean>(P, l_is_cat, (c + 1) & 3, 1, nb);
-      }
-      float v[8];
-      tmem_ld8(d_tmem + 64 * c + T.kcol, v);
-      epi_sub<EPI, kPasses, kLean, kNE>(args, T, P, oa, v, c, 0, l, l_is_cat, train, store_state, last_step, sbar, acc);
-      tmem_ld8(d_tmem + 64 * c + T.kcol + 8, v);
-      epi_sub<EPI, kPasses, kLean, kNE>(args, T, P, ob, v, c, 1, l, l_is_cat, train, store_state, last_step, sbar, acc);
-      if (chunk_release) {
-        fence_proxy_async_smem();
-        __syncwarp();
-        if (lane == 0) mbar_arrive(smem_u32(&tail->a_ready[c]));
-      }
-      oa = na; ob = nb;
+  for (int ci = 0; ci < 4; ++ci) {
+    const int c = (ci + T.c0) & 3;
+    EpiOps na = oa, nb = ob;
+    if (ci < 3) {
+      epi_load<EPI, kPasses, kLean>(P, l_is_cat, (c + 1) & 3, 0, na);
+      epi_load<EPI, kPasses, kLean>(P, l_is_cat, (c + 1) & 3, 1, nb);
     }
-  } else {
-#pragma unroll 1
-    for (int ci = 0; ci < 4; ++ci) {
-      const int c = (ci + T.c0) & 3;
-      float v[8];
-      if (ABL(T.ablate, 128)) {           // DEV: barrier hand-off only (measures the MMA / weight-ring pipeline alone)
-        if (chunk_release) {
-          __syncwarp();
-          if (lane == 0) mbar_arrive(smem_u32(&tail->a_ready[c]));
-        }
-        continue;
-      }
-      epi_load<EPI, kPasses, kLean>(P, l_is_cat, c, 1, ob);
-      tmem_ld8(d_tmem + 64 * c + T.kcol, v);
-      epi_sub<EPI, kPasses, kLean, kNE>(args, T, P, oa, v, c, 0, l, l_is_cat, train, store_state, last_step, sbar, acc);
-      if (ci < 3) epi_load<EPI, kPasses, kLean>(P, l_is_cat, (c + 1) & 3, 0, oa);
-      tmem_ld8(d_tmem + 64 * c + T.kcol + 8, v);
-      epi_sub<EPI, kPasses, kLean, kNE>(args, T, P, ob, v, c, 1, l, l_is_cat, train, store_state, last_step, sbar, acc);
-      if (chunk_release) {
-        fence_proxy_async_smem();
-        __syncwarp();
-        if (lane == 0) mbar_arrive(smem_u32(&tail->a_ready[c]));
-      }
+    float v[8];
+    tmem_ld8(d_tmem + 64 * c + T.kcol, v);
+    epi_sub<EPI, kPasses, kLean, kNE>(args, T, P, oa, v, c, 0, l, l_is_cat, train, store_state, last_step, sbar, acc);
+    tmem_ld8(d_tmem + 64 * c + T.kcol + 8, v);
+    epi_sub<EPI, kPasses, kLean, kNE>(args, T, P, ob, v, c, 1, l, l_is_cat, train, store_state, last_step, sbar, acc);
+    if (chunk_release) {
+      fence_proxy_async_smem();
+      __syncwarp();
+      if (lane == 0) mbar_arrive(smem_u32(&tail->a_ready[c]));
     }
+    oa = na; ob = nb;
   }
   tc_fence_before();
 }
@@ -377,7 +330,7 @@ __device__ __forceinline__ void epi_step(const TcChainArgs& args, const EpiT& T,
 // kNE = embedding halves of 256 internal columns the program was built for (1: E <= 256 -- every shipped default
 // config; 2: E <= 512).  A template parameter so that the single-half kernel carries none of the second half's
 // run-time flag tests (they cost 2.6 % of the default workload's kernel time when they were run-time only).
-template <int kPasses, int kWide, bool kLean, int kNE>
+template <int kPasses, bool kLean, int kNE>
 __global__ void __launch_bounds__(NUM_THREADS, 1) tc_chain_kernel(const __grid_constant__ TcChainArgs args) {
   using Cfg = ChainCfg<kPasses>;
   extern __shared__ __align__(1024) uint8_t smem[];
@@ -403,7 +356,7 @@ __global__ void __launch_bounds__(NUM_THREADS, 1) tc_chain_kernel(const __grid_c
   tc_fence_after();
   const uint32_t tmem = tail->tmem_base;
 
-  const int rot = args.stagger ? (int)(blockIdx.x & 15u) : 0;
+  const int rot = (int)(blockIdx.x & 15u);
   const int my_tiles = (args.n_tiles > (int)blockIdx.x) ? (args.n_tiles - 1 - (int)blockIdx.x) / (int)gridDim.x + 1 : 0;
 
   // (setmaxnreg sits INSIDE each role branch: ptxas budgets registers per branch only when the re-allocation
@@ -419,7 +372,7 @@ __global__ void __launch_bounds__(NUM_THREADS, 1) tc_chain_kernel(const __grid_c
         const int tile = args.tile0 + blockIdx.x + it * gridDim.x;
         for (int s = 0; s < n_steps; ++s) {
           const TcStep st = args.steps[s];
-          if (args.prefetch && s + 1 < n_steps) {
+          if (s + 1 < n_steps) {
             // pull the side arrays the NEXT step's epilogue will read from HBM into L2 while this step runs
             const TcStep nx = args.steps[s + 1];
             const float* aux_t = args.aux + (size_t)tile * TC_TILE_FLOATS;
@@ -454,12 +407,10 @@ __global__ void __launch_bounds__(NUM_THREADS, 1) tc_chain_kernel(const __grid_c
             mbar_wait(smem_u32(&tail->w_empty[stage]), ph ^ 1);
             const uint32_t bar = smem_u32(&tail->w_full[stage]);
             const uint32_t dst = smem_u32(w_ring + stage * Cfg::kStageBytes);
-            if (ABL(args.ablate, 512)) { mbar_arrive(bar); continue; }      // DEV: no weight traffic at all
             const int kse = rot_kstep(ks, rot);
-            const bool blo = kPasses == 3 && !(st.flags & STF_NO_BLO);
-            mbar_arrive_expect_tx(bar, blo ? Cfg::kStageBytes : KSTEP_IMG_BYTES);
+            mbar_arrive_expect_tx(bar, Cfg::kStageBytes);
             bulk_g2s(dst, img_hi + (size_t)kse * KSTEP_IMG_BYTES, KSTEP_IMG_BYTES, bar);
-            if (blo) bulk_g2s(dst + KSTEP_IMG_BYTES, img_lo + (size_t)kse * KSTEP_IMG_BYTES, KSTEP_IMG_BYTES, bar);
+            if (kPasses == 3) bulk_g2s(dst + KSTEP_IMG_BYTES, img_lo + (size_t)kse * KSTEP_IMG_BYTES, KSTEP_IMG_BYTES, bar);
           }
         }
       }
@@ -472,7 +423,6 @@ __global__ void __launch_bounds__(NUM_THREADS, 1) tc_chain_kernel(const __grid_c
     for (int it = 0; it < my_tiles; ++it) {
       for (int s = 0; s < n_steps; ++s, ++n) {
         const uint32_t d_tmem = tmem + (n & 1) * 256;
-        const bool blo = !(args.steps[s].flags & STF_NO_BLO);
         for (int ks = 0; ks < N_KSTEPS; ++ks, ++j) {
           const int kse = rot_kstep(ks, rot);
           if ((ks & 3) == 0) mbar_wait(smem_u32(&tail->a_ready[kse >> 2]), n & 1);
@@ -483,12 +433,12 @@ __global__ void __launch_bounds__(NUM_THREADS, 1) tc_chain_kernel(const __grid_c
             const uint32_t b_base = smem_u32(w_ring + stage * Cfg::kStageBytes);
             const uint64_t ah = umma_desc(smem_u32(a_hi) + kse * 2 * A_LBO, A_LBO, 128);
             const uint64_t bh = umma_desc(b_base, B_LBO, 128);
-            if (!ABL(args.ablate, 256)) tc_mma_f16(d_tmem, ah, bh, idesc, ks != 0);
-            if (kPasses == 3 && !ABL(args.ablate, 256)) {
+            tc_mma_f16(d_tmem, ah, bh, idesc, ks != 0);
+            if (kPasses == 3) {
               const uint64_t al = umma_desc(smem_u32(a_lo) + kse * 2 * A_LBO, A_LBO, 128);
               const uint64_t bl = umma_desc(b_base + KSTEP_IMG_BYTES, B_LBO, 128);
               tc_mma_f16(d_tmem, al, bh, idesc, 1);
-              if (blo) tc_mma_f16(d_tmem, ah, bl, idesc, 1);
+              tc_mma_f16(d_tmem, ah, bl, idesc, 1);
             }
             tc_commit(smem_u32(&tail->w_empty[stage]));
             if (ks == N_KSTEPS - 1) tc_commit(smem_u32(&tail->d_full[n & 1]));
@@ -519,7 +469,7 @@ __global__ void __launch_bounds__(NUM_THREADS, 1) tc_chain_kernel(const __grid_c
       const int64_t pl = (int64_t)tile * TC_TILE + p;             // point index inside the chunk
       const bool real = pl < args.n_points;
       EpiT T;
-      T.p = p; T.kcol = 16 * jg; T.ablate = args.ablate; T.c0 = rot >> 2;
+      T.p = p; T.kcol = 16 * jg; T.c0 = rot >> 2;
       T.a_hi = a_hi + p * 16 + (2 * jg) * A_LBO;
       T.a_lo = a_lo + p * 16 + (2 * jg) * A_LBO;
       const size_t dthr = (size_t)tile * TC_DWL_TILE_BYTES + (size_t)(p >> 4) * 8192u + (size_t)(p & 15) * 16u + (size_t)(2 * jg) * 256u;
@@ -536,7 +486,6 @@ __global__ void __launch_bounds__(NUM_THREADS, 1) tc_chain_kernel(const __grid_c
         if (lane == 0) mbar_arrive(smem_u32(&tail->a_ready[c]));
       };
 
-      if (args.dbg_clock && blockIdx.x == 0 && threadIdx.x == 0 && it == 0) args.dbg_clock[120] = clock64();
       // ---------------- PE stage: x -> e (A operand of the first step) ----------------
       float xs[3] = {0.f, 0.f, 0.f};
       if (real) {
@@ -593,7 +542,7 @@ __global__ void __launch_bounds__(NUM_THREADS, 1) tc_chain_kernel(const __grid_c
             v[jj] = va; v[jj + 1] = vb;
           }
           put8<kPasses, kLean>(T, v, c, h, true, train ? (eh ? args.arr_yh_e1 : args.arr_yh) : -1);
-          if (store_state && !ABL(args.ablate, 2)) {
+          if (store_state) {
             st4(e32_h + sub_x(c, h), v[0], v[1], v[2], v[3]);
             st4(e32_h + sub_x(c, h) + 512, v[4], v[5], v[6], v[7]);
           }
@@ -619,9 +568,7 @@ __global__ void __launch_bounds__(NUM_THREADS, 1) tc_chain_kernel(const __grid_c
           for (int jj = 0; jj < 8; jj += 2) {
             const int k = k0 + jj;
             float va = 0.f, vb = 0.f;
-            if (ABL(args.ablate, 64)) {
-              va = u3[0];
-            } else if (k < two_half) {       // abar_e = (u . D_d) 2^f (cos, -sin)
+            if (k < two_half) {       // abar_e = (u . D_d) 2^f (cos, -sin)
               const int pi = k >> 1, d = args.pair_d[pi];
               const float ud = (u3[0] * c_ico[d][0] + u3[1] * c_ico[d][1] + u3[2] * c_ico[d][2]) * (float)(1 << args.pair_f[pi]);
               va = ud * ev[jj + 1];
@@ -639,8 +586,6 @@ __global__ void __launch_bounds__(NUM_THREADS, 1) tc_chain_kernel(const __grid_c
       };
       write_e_half(0);
 
-      const bool dbg = args.dbg_clock && blockIdx.x == 0 && threadIdx.x == 0 && it == 0;
-      if (dbg) args.dbg_clock[0] = clock64();
       EpiAcc gacc = {0.f, 0.f, 0.f, 0.f};                 // d sdf / d x_s partial sums over this thread's embedding columns
 
       for (int s = 0; s < n_steps; ++s, ++n) {
@@ -662,25 +607,22 @@ __global__ void __launch_bounds__(NUM_THREADS, 1) tc_chain_kernel(const __grid_c
         P.wout = Wp + args.wout_off;
         P.hlast = T.aux + (size_t)args.arr_hlast * T.aux_stride;
         P.e32 = (kNE == 2) ? e32_w + (size_t)st.eh * args.aux_stride : e32_w;
-        P.ablate = args.ablate;
         P.flags = st.flags;
         P.ecol0 = 256 * st.eh;
         EpiAcc acc_local = {0.f, 0.f, 0.f, 0.f};
         if (epi == EPI_S2_END && (kNE == 1 || (st.flags & STF_END_FIRST))) gacc = acc_local;
         EpiAcc& acc = (epi == EPI_S2_END) ? gacc : acc_local;
-        if (dbg) args.dbg_clock[1 + 2 * s] = clock64();
         switch (epi) {
-          case EPI_RAW:     epi_step<EPI_RAW, kPasses, kWide, kLean, kNE>(args, T, P, tail, d_tmem, n, l, train, store_state, last_step, sbar, acc, lane); break;
-          case EPI_S1:      epi_step<EPI_S1, kPasses, kWide, kLean, kNE>(args, T, P, tail, d_tmem, n, l, train, store_state, last_step, sbar, acc, lane); break;
-          case EPI_S1_LAST: epi_step<EPI_S1_LAST, kPasses, kWide, kLean, kNE>(args, T, P, tail, d_tmem, n, l, train, store_state, last_step, sbar, acc, lane); break;
-          case EPI_S2:      epi_step<EPI_S2, kPasses, kWide, kLean, kNE>(args, T, P, tail, d_tmem, n, l, train, store_state, last_step, sbar, acc, lane); break;
-          case EPI_S2_END:  epi_step<EPI_S2_END, kPasses, kWide, kLean, kNE>(args, T, P, tail, d_tmem, n, l, train, store_state, last_step, sbar, acc, lane); break;
-          case EPI_S3:      epi_step<EPI_S3, kPasses, kWide, kLean, kNE>(args, T, P, tail, d_tmem, n, l, train, store_state, last_step, sbar, acc, lane); break;
-          case EPI_S3_LAST: epi_step<EPI_S3_LAST, kPasses, kWide, kLean, kNE>(args, T, P, tail, d_tmem, n, l, train, store_state, last_step, sbar, acc, lane); break;
-          default:          epi_step<EPI_S4, kPasses, kWide, kLean, kNE>(args, T, P, tail, d_tmem, n, l, train, store_state, last_step, sbar, acc, lane); break;
+          case EPI_RAW:     epi_step<EPI_RAW, kPasses, kLean, kNE>(args, T, P, tail, d_tmem, n, l, train, store_state, last_step, sbar, acc, lane); break;
+          case EPI_S1:      epi_step<EPI_S1, kPasses, kLean, kNE>(args, T, P, tail, d_tmem, n, l, train, store_state, last_step, sbar, acc, lane); break;
+          case EPI_S1_LAST: epi_step<EPI_S1_LAST, kPasses, kLean, kNE>(args, T, P, tail, d_tmem, n, l, train, store_state, last_step, sbar, acc, lane); break;
+          case EPI_S2:      epi_step<EPI_S2, kPasses, kLean, kNE>(args, T, P, tail, d_tmem, n, l, train, store_state, last_step, sbar, acc, lane); break;
+          case EPI_S2_END:  epi_step<EPI_S2_END, kPasses, kLean, kNE>(args, T, P, tail, d_tmem, n, l, train, store_state, last_step, sbar, acc, lane); break;
+          case EPI_S3:      epi_step<EPI_S3, kPasses, kLean, kNE>(args, T, P, tail, d_tmem, n, l, train, store_state, last_step, sbar, acc, lane); break;
+          case EPI_S3_LAST: epi_step<EPI_S3_LAST, kPasses, kLean, kNE>(args, T, P, tail, d_tmem, n, l, train, store_state, last_step, sbar, acc, lane); break;
+          default:          epi_step<EPI_S4, kPasses, kLean, kNE>(args, T, P, tail, d_tmem, n, l, train, store_state, last_step, sbar, acc, lane); break;
         }
 
-        if (dbg) args.dbg_clock[2 + 2 * s] = clock64();
         if (kNE == 2 && epi == EPI_RAW) {
           // second embedding half of a wide embedding: its A operand replaces the first half's (whose products are done)
           if (st.flags & STF_PE_E) write_e_half(st.peh);
@@ -780,42 +722,38 @@ __global__ void __launch_bounds__(NUM_THREADS, 1) tc_chain_kernel(const __grid_c
   if (warp == EPI_WARPS) tmem_dealloc(tmem, 512);
 }
 
-template <int kPasses, int kWide, bool kLean, int kNE>
+template <int kPasses, bool kLean, int kNE>
 static void chain_launch_t(const TcChainArgs& args, int grid, cudaStream_t st) {
-  tc_chain_kernel<kPasses, kWide, kLean, kNE><<<grid, NUM_THREADS, ChainCfg<kPasses>::kSmem, st>>>(args);
+  tc_chain_kernel<kPasses, kLean, kNE><<<grid, NUM_THREADS, ChainCfg<kPasses>::kSmem, st>>>(args);
 }
 
 int tc_chain_launch(isdfb_ctx* ctx, const TcChainArgs& args, int passes, int grid, cudaStream_t st) {
-  const bool two = args.n_eh == 2;       // wide embeddings: always the 16-column-TMEM-load epilogue variant
+  const bool two = args.n_eh == 2;
   if (passes == 3) {
-    if (args.lean) { if (two) chain_launch_t<3, 1, true, 2>(args, grid, st); else chain_launch_t<3, 1, true, 1>(args, grid, st); }
-    else if (two) chain_launch_t<3, 1, false, 2>(args, grid, st);
-    else if (args.wide) chain_launch_t<3, 1, false, 1>(args, grid, st);
-    else chain_launch_t<3, 0, false, 1>(args, grid, st);
+    if (args.lean) { if (two) chain_launch_t<3, true, 2>(args, grid, st); else chain_launch_t<3, true, 1>(args, grid, st); }
+    else if (two) chain_launch_t<3, false, 2>(args, grid, st);
+    else chain_launch_t<3, false, 1>(args, grid, st);
   } else {
-    if (two) chain_launch_t<1, 1, false, 2>(args, grid, st);
-    else if (args.wide) chain_launch_t<1, 1, false, 1>(args, grid, st);
-    else chain_launch_t<1, 0, false, 1>(args, grid, st);
+    if (two) chain_launch_t<1, false, 2>(args, grid, st);
+    else chain_launch_t<1, false, 1>(args, grid, st);
   }
   ISDFB_LAUNCHED(ctx);
   ISDFB_CUDA_OK(ctx, cudaGetLastError());
   return ISDFB_OK;
 }
 
-template <int kPasses, int kWide, bool kLean, int kNE>
+template <int kPasses, bool kLean, int kNE>
 static cudaError_t chain_attr_t() {
-  return cudaFuncSetAttribute(tc_chain_kernel<kPasses, kWide, kLean, kNE>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+  return cudaFuncSetAttribute(tc_chain_kernel<kPasses, kLean, kNE>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                               ChainCfg<kPasses>::kSmem);
 }
 
 int tc_chain_init(isdfb_ctx* ctx) {
-  ISDFB_CUDA_OK(ctx, (chain_attr_t<3, 0, false, 1>()));
-  ISDFB_CUDA_OK(ctx, (chain_attr_t<3, 1, false, 1>()));
-  ISDFB_CUDA_OK(ctx, (chain_attr_t<3, 1, false, 2>()));
-  ISDFB_CUDA_OK(ctx, (chain_attr_t<3, 1, true, 1>()));
-  ISDFB_CUDA_OK(ctx, (chain_attr_t<3, 1, true, 2>()));
-  ISDFB_CUDA_OK(ctx, (chain_attr_t<1, 0, false, 1>()));
-  ISDFB_CUDA_OK(ctx, (chain_attr_t<1, 1, false, 1>()));
-  ISDFB_CUDA_OK(ctx, (chain_attr_t<1, 1, false, 2>()));
+  ISDFB_CUDA_OK(ctx, (chain_attr_t<3, false, 1>()));
+  ISDFB_CUDA_OK(ctx, (chain_attr_t<3, false, 2>()));
+  ISDFB_CUDA_OK(ctx, (chain_attr_t<3, true, 1>()));
+  ISDFB_CUDA_OK(ctx, (chain_attr_t<3, true, 2>()));
+  ISDFB_CUDA_OK(ctx, (chain_attr_t<1, false, 1>()));
+  ISDFB_CUDA_OK(ctx, (chain_attr_t<1, false, 2>()));
   return ISDFB_OK;
 }

@@ -14,9 +14,7 @@ enum {
   STF_PE_E = 2,        // EPI_RAW: after the drain write the embedding half `peh` into A (S1)
   STF_PE_ABAR = 4,     // EPI_RAW: after the drain write the adjoint abar_e half `peh` into A (S3)
   STF_END_FIRST = 8,   // EPI_S2_END: first embedding half -> reset the d sdf/dx accumulators
-  STF_END_LAST = 16,   // EPI_S2_END: last embedding half -> reduce, loss, then abar_e half 0 into A
-  STF_NO_BLO = 32      // experiment (ISDFB_GRAD_2PASS): skip the A_hi * B_lo pass of this product (gradient-only sweeps S3 / S4):
-                       // the weights enter as single bf16, only their hi image is streamed
+  STF_END_LAST = 16    // EPI_S2_END: last embedding half -> reduce, loss, then abar_e half 0 into A
 };
 struct TcStep {
   int32_t unit;     // weight unit (tc_pack.cu)
@@ -47,12 +45,6 @@ struct TcChainArgs {
   int32_t n_steps, mode, L, ic, E, S;
   int32_t n_tiles;           // tiles processed by this launch ...
   int32_t tile0;             // ... starting at this tile of the chunk
-  int32_t prefetch;          // 1: bulk-prefetch the next step's side arrays into L2 (producer warp)
-  int32_t stagger;           // 1: per-CTA rotation of the K order (rot_kstep) against L2 hot-spotting on the weights
-  int32_t wide;              // 1: epilogue variant with 16-column TMEM loads (two interleaved chains per chunk)
-  int32_t ablate;            // DEV ONLY (env ISDFB_ABLATE + a build with -DISDFB_DEV_ABLATE; results invalid): 1 no dW-layout stores, 2 no aux stores,
-                             // 4 no sigma stores, 8 no side loads, 16 relu instead of softplus, 32 no A-image stores,
-                             // 64 no PE-Jacobian / abar_e math -- timing ablations for profiles/
   int64_t n_points;          // real points in this chunk
   int64_t p0;                // global index of the chunk's first point (sample index r*S+j)
   PEParams pe;
@@ -89,7 +81,6 @@ struct TcChainArgs {
   int32_t arr_yh, arr_ya, arr_xd, arr_xz, arr_v;            // dW-layout array indices
   int32_t arr_yh_e1, arr_ya_e1;                             // dW-layout arrays of the second embedding half (e, abar_e)
   int32_t n_eh;                                             // embedding halves (1: E <= 256, 2: E <= 512)
-  long long* dbg_clock;                                     // optional: per-step timeline of CTA 0 (tests)
   uint8_t pair_d[TC_MAX_EH * TC_H / 2], pair_f[TC_MAX_EH * TC_H / 2];   // internal PE column pair -> (direction, octave)
 };
 

@@ -102,7 +102,7 @@ __global__ void __launch_bounds__(DW_THREADS, 1) tc_dw_kernel(const TcDwArgs arg
               if (kPasses == 3) {
                 const uint64_t bl = umma_desc(base + Cfg::kXBytes + 8192, 128, 256);
                 tc_mma_f16(tmem, al, bh, idesc_main, 1);
-                if (!args.skip_ylo) tc_mma_f16(tmem, ah, bl, idesc_main, 1);
+                tc_mma_f16(tmem, ah, bl, idesc_main, 1);
               }
             }
             if (pr.ones) {

@@ -1,7 +1,6 @@
 // Host orchestration of the tensor-core path: state, step programs, weight-gradient jobs, launches.
 #include "tc_path.cuh"
 #include <new>
-#include <stdlib.h>
 
 static TcStep& add_step(TcChainArgs& a, int unit, int orient, int epi, int layer, int aux = 0) {
   TcStep& s = a.steps[a.n_steps++];
@@ -61,12 +60,6 @@ static void build_program(const ModelLayout& lay, int mode, int NE, TcChainArgs&
   }
   // ---- S4 (reverse; the two d / d e products are not needed)
   for (int l = L - 1; l >= 1; --l) add_step(a, l, 1, EPI_S4, l - 1);
-  if (getenv("ISDFB_GRAD_2PASS"))          // experiment: weights as single bf16 in the gradient-only sweeps
-    for (int s = 0; s < a.n_steps; ++s)
-      if (a.steps[s].epi == EPI_S3 || a.steps[s].epi == EPI_S3_LAST || a.steps[s].epi == EPI_S4 ||
-          (a.steps[s].epi == EPI_RAW && a.steps[s].aux != PART_CAT_S1 && a.steps[s].aux != PART_CAT_S2 &&
-           a.steps[s].aux != PART_CAT_S2_H1 && a.steps[s].aux != PART_L0_S1))
-        a.steps[s].flags |= STF_NO_BLO;
 }
 
 // Host-only view of the step program (no CUDA call, no context): what the chain kernel will run for a model shape.
@@ -168,21 +161,12 @@ int tc_create(isdfb_ctx* ctx) {
 
   ISDFB_CUDA_OK(ctx, cudaMalloc(&tc->dw_counters, TC_MAX_JOBS * sizeof(int32_t)));
   ISDFB_CUDA_OK(ctx, cudaMemset(tc->dw_counters, 0, TC_MAX_JOBS * sizeof(int32_t)));
-  if (getenv("ISDFB_DEBUG_CLOCK")) {
-    ISDFB_CUDA_OK(ctx, cudaMalloc(&tc->dbg_clock, 128 * sizeof(long long)));
-    ISDFB_CUDA_OK(ctx, cudaMemset(tc->dbg_clock, 0, 128 * sizeof(long long)));
-  }
   for (int mode = 0; mode < 3; ++mode) {
     TcChainArgs& a = tc->proto[mode];
     memset(&a, 0, sizeof(a));
     build_program(lay, mode, NE, a);
     a.n_eh = NE;
     a.mode = mode; a.L = L; a.ic = ic; a.E = lay.E;
-    a.prefetch = getenv("ISDFB_NO_PREFETCH") ? 0 : 1;
-    a.stagger = getenv("ISDFB_STAGGER") ? atoi(getenv("ISDFB_STAGGER")) : 1;
-    a.wide = getenv("ISDFB_EPI_WIDE") ? atoi(getenv("ISDFB_EPI_WIDE")) : 1;
-    a.ablate = getenv("ISDFB_ABLATE") ? atoi(getenv("ISDFB_ABLATE")) : 0;
-    a.dbg_clock = tc->dbg_clock;
     a.pe = ctx->pe;
     a.scale_output = ctx->cfg.scale_output;
     a.w_img = tc->w_img;
@@ -196,7 +180,6 @@ int tc_create(isdfb_ctx* ctx) {
     a.arr_part = 0; a.arr_e32 = n_part; a.arr_hlast = n_part + NE; a.arr_zb2 = n_part + NE + 1;   // zbar2 (fp32): absent in lean mode
     a.lean = lean ? 1 : 0;
     a.zb2h = lean ? tc->sig16 + tc->dwl_stride * L : nullptr;
-    if (lean) a.wide = 1;
     for (int i = 0; i < TC_MAX_EH * TC_H / 2; ++i) {      // pair i = (direction, octave) of internal columns 2i, 2i+1
       a.pair_d[i] = (uint8_t)(i < pe_half ? i / lay.n_freqs : 0);
       a.pair_f[i] = (uint8_t)(i < pe_half ? i % lay.n_freqs : 0);
@@ -243,7 +226,6 @@ int tc_create(isdfb_ctx* ctx) {
   d.g_packed = ctx->g_packed;
   d.wout_off = lay.wout_off;
   d.scale_output = ctx->cfg.scale_output;
-  d.skip_ylo = getenv("ISDFB_DW_SKIP_YLO") ? 1 : 0;
   return ISDFB_OK;
 }
 
@@ -268,28 +250,72 @@ static inline int passes_of(const isdfb_ctx* ctx) {
 // the weight-gradient kernel reads single-bf16 operands in lean mode
 static inline int dw_passes_of(const isdfb_ctx* ctx) { return ctx->cfg.precision == ISDFB_PREC_BF16X3 ? 3 : 1; }
 
+// A call over n points runs in chunks of at most cap points (the side state is sized for cap points): chunk
+// [p0, p0 + nc) for p0 = 0, cap, 2 cap, ..., cut into tiles of TC_TILE points.  f(p0, nc, tiles) runs once per chunk,
+// in order; a non-zero return stops the walk and is returned.
+template <class F>
+static int for_each_chunk(int64_t n, int64_t cap, F&& f) {
+  for (int64_t p0 = 0; p0 < n; p0 += cap) {
+    const int64_t nc = (n - p0 < cap) ? (n - p0) : cap;
+    const int rc = f(p0, nc, (int)((nc + TC_TILE - 1) / TC_TILE));
+    if (rc) return rc;
+  }
+  return ISDFB_OK;
+}
+
+// The launches of one training chunk.  A wave runs the chain kernel over tiles [tile0, tile0 + n_tiles) on chain_grid
+// CTAs and then the weight-gradient kernel over the same tiles on dw_grid CTAs, on the side stream when dw_side.
+struct TcWave { int tile0, n_tiles, chain_grid, dw_grid; bool dw_side; };
+struct TcChunkPlan { int n_waves; TcWave wave[2]; };
+
+// A chunk of more than one and less than two waves of tiles runs as two waves when overlap is allowed: the weight
+// gradients of the full wave 1 run on the side stream underneath the partial wave 2, on the CTAs wave 2 leaves idle --
+// but never fewer than one CTA per job: tc_dw_kernel maps CTA b to job b % n_jobs, so the jobs past a smaller grid
+// would get no CTA and their gradient over wave 1 would be lost.  Otherwise one wave: the chain on at most num_sms
+// persistent CTAs, then the dW on num_sms CTAs.
+static TcChunkPlan chunk_plan(int tiles, int num_sms, int n_jobs, bool overlap) {
+  TcChunkPlan pl;
+  if (overlap && tiles > num_sms && tiles < 2 * num_sms) {
+    const int rest = tiles - num_sms, idle = num_sms - rest;
+    pl.n_waves = 2;
+    pl.wave[0] = {0, num_sms, num_sms, idle > n_jobs ? idle : n_jobs, true};
+    pl.wave[1] = {num_sms, rest, rest, num_sms, false};
+  } else {
+    pl.n_waves = 1;
+    pl.wave[0] = {0, tiles, tiles < num_sms ? tiles : num_sms, num_sms, false};
+  }
+  return pl;
+}
+
+// Arrivals at job j's counter from one weight-gradient launch of `grid` CTAs (grid >= n_jobs) over `tiles` tiles:
+// tc_dw_kernel maps CTA b to job b % n_jobs and tile split b / n_jobs, so job j has (grid - 1 - j) / n_jobs + 1 splits,
+// and only a split that owns at least one tile arrives.
+static inline int dw_arrivals(int j, int grid, int tiles, int n_jobs) {
+  const int n_splits = (grid - 1 - j) / n_jobs + 1;
+  return n_splits < tiles ? n_splits : tiles;
+}
+
 static int tc_forward_impl(isdfb_ctx* ctx, const float* x, const float* noise, float noise_std, int64_t n, float* sdf,
                            float* grad, cudaStream_t st, const TcGrid* grid) {
   TcState* tc = reinterpret_cast<TcState*>(ctx->tc);
-  for (int64_t p0 = 0; p0 < n; p0 += ctx->cap) {
-    const int64_t nc = (n - p0 < ctx->cap) ? (n - p0) : ctx->cap;
+  return for_each_chunk(n, ctx->cap, [&](int64_t p0, int64_t nc, int tiles) -> int {
     TcChainArgs a = tc->proto[grad ? TC_MODE_FWD_GRAD : TC_MODE_FWD];
     if (grid) a.grid = *grid;
     a.n_points = nc;
-    a.n_tiles = (int)((nc + TC_TILE - 1) / TC_TILE);
+    a.n_tiles = tiles;
     a.p0 = p0;
     a.x = x ? x + p0 * 3 : nullptr;
     a.noise = noise ? noise + p0 : nullptr;
     a.noise_std = noise_std;
     a.sdf_out = sdf + p0;
     a.g_out = grad ? grad + p0 * 3 : nullptr;
-    const int n_cta = a.n_tiles < tc->num_sms ? a.n_tiles : tc->num_sms;
+    const TcWave w = chunk_plan(tiles, tc->num_sms, tc->dw.n_jobs, false).wave[0];
     const int pi = prof_begin(tc, st);
-    int rc = tc_chain_launch(ctx, a, passes_of(ctx), n_cta, st);
+    const int rc = tc_chain_launch(ctx, a, passes_of(ctx), w.chain_grid, st);
     if (rc) return rc;
     prof_mark(tc, pi, 1, st);
-  }
-  return ISDFB_OK;
+    return ISDFB_OK;
+  });
 }
 
 int tc_forward(isdfb_ctx* ctx, const float* x, const float* noise, float noise_std, int64_t n, float* sdf,
@@ -313,49 +339,28 @@ int tc_forward_grid(isdfb_ctx* ctx, const float* lin, int dim, const float* scal
   return tc_forward_impl(ctx, nullptr, nullptr, 0.f, (int64_t)dim * dim * dim, sdf, nullptr, st, &g);
 }
 
-// Grid of the wave-1 weight-gradient launch of a two-wave chunk (tiles = num_sms + rest): the CTAs the partial wave 2
-// leaves idle, but never fewer than one CTA per job -- tc_dw_kernel maps CTA b to job b % n_jobs, so a smaller grid
-// would leave jobs n_jobs-grid.. without a CTA and their gradient over the first num_sms tiles would be lost.  The
-// launch and the exchange's expected-arrival counts both take the grid from here.
-static inline int dw_wave1_grid(const TcState* tc, int rest) {
-  const int idle = tc->num_sms - rest;
-  return idle > tc->dw.n_jobs ? idle : tc->dw.n_jobs;
-}
-
 int tc_train(isdfb_ctx* ctx, const float* pc, const float* z_vals, const float* depth_sample, const float* dirs_C,
              const float* T_WC_sample, const float* norm_sample, const float* noise, const uint8_t* ray_valid,
              int64_t n_rays, int32_t S, const isdfb_loss_cfg* loss, float* sdf, float* grad, float* loss_mat,
              float* loss_sums, cudaStream_t st) {
   TcState* tc = reinterpret_cast<TcState*>(ctx->tc);
   const int64_t n = n_rays * S;
-  const bool two_wave_ok = !tc->profiling && !getenv("ISDFB_NO_OVERLAP");
-  // weight-gradient launches of this step as (grid, tiles): with a gradient exchange installed the last CTA of
-  // each job over ALL of them forwards the job's tile to the multicast buffer, so it must know how many arrive
+  const int n_jobs = tc->dw.n_jobs;
+  // kernel timing reads one (chain, dW) event pair per chunk, so profiling runs every chunk as one wave
+  const bool overlap = !tc->profiling;
+  // with a gradient exchange installed the last CTA of each job over ALL weight-gradient launches of the step
+  // forwards the job's tile to the multicast buffer, so it must know how many arrive
   int32_t expect[TC_MAX_JOBS] = {0};
-  if (ctx->g_xchg) {
-    auto plan = [&](int grid, int tiles) {
-      for (int j = 0; j < tc->dw.n_jobs; ++j) {
-        const int n_splits = (grid - 1 - j) / tc->dw.n_jobs + 1;
-        expect[j] += n_splits < tiles ? n_splits : tiles;
-      }
-    };
-    for (int64_t p0 = 0; p0 < n; p0 += ctx->cap) {
-      const int64_t nc = (n - p0 < ctx->cap) ? (n - p0) : ctx->cap;
-      const int tiles = (int)((nc + TC_TILE - 1) / TC_TILE);
-      if (tiles > tc->num_sms && tiles < 2 * tc->num_sms && two_wave_ok) {
-        const int rest = tiles - tc->num_sms;
-        plan(dw_wave1_grid(tc, rest), tc->num_sms);
-        plan(tc->num_sms, rest);
-      } else {
-        plan(tc->num_sms, tiles);
-      }
-    }
-  }
-  for (int64_t p0 = 0; p0 < n; p0 += ctx->cap) {
-    const int64_t nc = (n - p0 < ctx->cap) ? (n - p0) : ctx->cap;
+  if (ctx->g_xchg)
+    for_each_chunk(n, ctx->cap, [&](int64_t, int64_t, int tiles) -> int {
+      const TcChunkPlan pl = chunk_plan(tiles, tc->num_sms, n_jobs, overlap);
+      for (int w = 0; w < pl.n_waves; ++w)
+        for (int j = 0; j < n_jobs; ++j) expect[j] += dw_arrivals(j, pl.wave[w].dw_grid, pl.wave[w].n_tiles, n_jobs);
+      return ISDFB_OK;
+    });
+  return for_each_chunk(n, ctx->cap, [&](int64_t p0, int64_t nc, int tiles) -> int {
     TcChainArgs a = tc->proto[TC_MODE_TRAIN];
     a.n_points = nc;
-    a.n_tiles = (int)((nc + TC_TILE - 1) / TC_TILE);
     a.p0 = p0;
     a.S = S;
     a.loss = *loss;
@@ -370,46 +375,36 @@ int tc_train(isdfb_ctx* ctx, const float* pc, const float* z_vals, const float* 
     a.loss_sums = loss_sums;
     a.g_packed = ctx->g_xchg ? ctx->g_mc[ctx->g_sel] : ctx->g_packed;
     a.g_mc = ctx->g_xchg ? 1 : 0;
-    const int total_tiles = a.n_tiles;
-    const int pi = prof_begin(tc, st);
     TcDwArgs d = tc->dw;
     d.g_mc = ctx->g_xchg ? 1 : 0;
     d.g_packed = ctx->g_xchg ? ctx->g_own : ctx->g_packed;      // exchange: accumulate in the local stage ...
     d.g_mc_out = ctx->g_xchg ? ctx->g_mc[ctx->g_sel] : nullptr; // ... the last CTA per job forwards it
     d.counters = tc->dw_counters;
     for (int j = 0; j < TC_MAX_JOBS; ++j) d.expect[j] = expect[j];
-    int rc;
-    if (total_tiles > tc->num_sms && total_tiles < 2 * tc->num_sms && two_wave_ok) {
-      // two waves: the weight gradients of wave 1 run on a side stream underneath the (partial) wave 2
-      a.tile0 = 0; a.n_tiles = tc->num_sms;
-      rc = tc_chain_launch(ctx, a, passes_of(ctx), tc->num_sms, st);
-      if (rc) return rc;
-      ISDFB_CUDA_OK(ctx, cudaEventRecord(tc->ev_fork, st));
-      ISDFB_CUDA_OK(ctx, cudaStreamWaitEvent(tc->side, tc->ev_fork, 0));
-      d.tile0 = 0; d.n_tiles = tc->num_sms;
-      const int rest = total_tiles - tc->num_sms;
-      rc = tc_dw_launch(ctx, d, dw_passes_of(ctx), dw_wave1_grid(tc, rest), tc->side);
-      if (rc) return rc;
-      ISDFB_CUDA_OK(ctx, cudaEventRecord(tc->ev_join, tc->side));
-      a.tile0 = tc->num_sms; a.n_tiles = rest;
-      rc = tc_chain_launch(ctx, a, passes_of(ctx), rest, st);
-      if (rc) return rc;
-      ISDFB_CUDA_OK(ctx, cudaStreamWaitEvent(st, tc->ev_join, 0));
-      d.tile0 = tc->num_sms; d.n_tiles = rest;
-      rc = tc_dw_launch(ctx, d, dw_passes_of(ctx), tc->num_sms, st);
-      if (rc) return rc;
-    } else {
-      const int grid = a.n_tiles < tc->num_sms ? a.n_tiles : tc->num_sms;
-      rc = tc_chain_launch(ctx, a, passes_of(ctx), grid, st);
+    const TcChunkPlan pl = chunk_plan(tiles, tc->num_sms, n_jobs, overlap);
+    const int pi = prof_begin(tc, st);                // -1 (marks are no-ops) unless profiling, which plans one wave
+    for (int w = 0; w < pl.n_waves; ++w) {
+      const TcWave& wv = pl.wave[w];
+      a.tile0 = d.tile0 = wv.tile0;
+      a.n_tiles = d.n_tiles = wv.n_tiles;
+      int rc = tc_chain_launch(ctx, a, passes_of(ctx), wv.chain_grid, st);
       if (rc) return rc;
       prof_mark(tc, pi, 1, st);
-      d.tile0 = 0; d.n_tiles = total_tiles;
-      rc = tc_dw_launch(ctx, d, dw_passes_of(ctx), tc->num_sms, st);
-      if (rc) return rc;
-      prof_mark(tc, pi, 2, st);
+      if (wv.dw_side) {                                // fork: these weight gradients run underneath the next wave
+        ISDFB_CUDA_OK(ctx, cudaEventRecord(tc->ev_fork, st));
+        ISDFB_CUDA_OK(ctx, cudaStreamWaitEvent(tc->side, tc->ev_fork, 0));
+        rc = tc_dw_launch(ctx, d, dw_passes_of(ctx), wv.dw_grid, tc->side);
+        if (rc) return rc;
+        ISDFB_CUDA_OK(ctx, cudaEventRecord(tc->ev_join, tc->side));
+      } else {
+        if (w > 0 && pl.wave[w - 1].dw_side) ISDFB_CUDA_OK(ctx, cudaStreamWaitEvent(st, tc->ev_join, 0));
+        rc = tc_dw_launch(ctx, d, dw_passes_of(ctx), wv.dw_grid, st);
+        if (rc) return rc;
+        prof_mark(tc, pi, 2, st);
+      }
     }
-  }
-  return ISDFB_OK;
+    return ISDFB_OK;
+  });
 }
 
 extern "C" int isdfb_debug_buffers(isdfb_ctx* ctx, float** aux, int64_t* aux_stride_floats, void** dwl_hi,
@@ -421,14 +416,6 @@ extern "C" int isdfb_debug_buffers(isdfb_ctx* ctx, float** aux, int64_t* aux_str
   *aux = tc->aux; *aux_stride_floats = (int64_t)tc->aux_stride;
   *dwl_hi = tc->dwl_hi; *dwl_lo = tc->dwl_lo; *dwl_stride_bytes = (int64_t)tc->dwl_stride;
   *n_aux = tc->n_aux; *n_dwl = tc->n_dwl; *tiles_cap = tc->tiles_cap; *sig16 = tc->sig16;
-  if (tc->dbg_clock) {   // debug timeline: printed by the host on request
-    long long h[128];
-    cudaMemcpy(h, tc->dbg_clock, sizeof(h), cudaMemcpyDeviceToHost);
-    const int ns = tc->proto[TC_MODE_TRAIN].n_steps;
-    printf("[isdfb] CTA0 tile0 timeline (cycles): PE took %lld; PE_end=0", h[0] - h[120]);
-    for (int s = 0; s < ns; ++s) printf(" | s%d epi%d wait_end=%lld epi_end=%lld", s, tc->proto[TC_MODE_TRAIN].steps[s].epi, h[1 + 2 * s] - h[0], h[2 + 2 * s] - h[0]);
-    printf("\n");
-  }
   return ISDFB_OK;
 }
 

@@ -22,7 +22,6 @@ struct TcDwJob {
 struct TcDwArgs {
   TcDwJob jobs[TC_MAX_JOBS];
   int32_t n_jobs, n_tiles, tile0;
-  int32_t skip_ylo;        // experiment: drop the X_hi*Y_lo pass (Y = layer inputs rounded to bf16)
   const uint8_t *dwl_hi, *dwl_lo;
   size_t dwl_stride;
   float* g_packed;         // where the TMEM accumulators are flushed (red.global.add): the gradient itself, or with an
@@ -54,7 +53,6 @@ struct TcState {
   int32_t* dw_counters;    // device, [TC_MAX_JOBS], zero between steps
   cudaStream_t side;       // second stream: weight gradients of the first wave overlap the second wave
   cudaEvent_t ev_fork, ev_join;
-  long long* dbg_clock;    // device buffer [128] when ISDFB_DEBUG_CLOCK is set
 };
 
 int tc_dw_launch(isdfb_ctx* ctx, const TcDwArgs& args, int passes, int grid, cudaStream_t st);
